@@ -79,17 +79,22 @@ def test_matrix_free_model_equals_assembled_operator():
         assert np.abs(y0 - y1).max() / np.abs(y0).max() < 1e-12
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("name", ["c1_64", "c1_64_sym_pmc_pec", "lossy_48", "nonuniform_56", "angled_48_minus", "offdiag_48", "c4_96"])
 def test_restatement_matches_live_reference(name):
+    """The reference's result is computed live where its source tree (or oracle/_ref) is present, else read from the golden
+    fixture it produced (tests/golden/make_golden.py: same inputs, same call)."""
     fac, kw, _ = CASES[name]
     wl = fac()
-    f0, n0, s0 = ref_shim.compute_modes(wl.eps_cross, wl.coords, wl.freqs[0], wl.mode_spec, **kw)
+    if ref_shim.available():
+        f0, n0, s0 = ref_shim.compute_modes(wl.eps_cross, wl.coords, wl.freqs[0], wl.mode_spec, **kw)
+        sig0 = signature(f0)
+    else:
+        g = load_golden(name)
+        n0, sig0, s0 = g["n_ref"], g["sig_ref"], str(g["spec"])
     f1, n1, s1 = R.compute_modes(wl.eps_cross, wl.coords, wl.freqs[0], wl.mode_spec, **kw)
     assert s0 == s1
     assert np.abs(n0 - n1).max() < 1e-10
-    assert np.abs(signature(f0) - signature(f1)).max() < 1e-5
+    assert np.abs(sig0 - signature(f1)).max() < 1e-5
 
 
 @pytest.mark.reference

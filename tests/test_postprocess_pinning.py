@@ -47,15 +47,18 @@ def _live():
     return ref_post.available()
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("name", list(PC.CASES))
 def test_restatement_against_the_live_reference(name):
-    if not _live():
-        pytest.skip("no reference tree here")
+    """On the seeded inputs: the reference's results are computed live where its source tree is present, else read from the
+    fixture it produced for these inputs (tests/golden/make_post_golden.py)."""
     c = PC.inputs(name)
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore", RuntimeWarning)
-        ref = PC.reference_results(c)
+    if _live():
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore", RuntimeWarning)
+            ref = PC.reference_results(c)
+    else:
+        z = np.load(os.path.join(GOLDEN, f"post_{name}.npz"))
+        ref = {k: z[f"ref_{k}"] for k in PC.KEYS}
     err = PC.compare(ref, PC.oracle_results(c), skip=PC.skipped_keys(c))
     assert max(err.values()) < TOL, err
 
