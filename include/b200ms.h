@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define B200MS_VERSION 203
+#define B200MS_VERSION 204
 
 /* return codes */
 enum {
@@ -188,41 +188,29 @@ typedef struct {
   double inner_relax_cap; /* loosest inner tolerance allowed (default 1e-4) */
   int gmres_cgs2;        /* inner FGMRES Gram-Schmidt: 1 always two passes (CGS2); 0 one pass (+ a second on cancellation; measured 3x more
                             iterations at tol 1e-10); 2 (default) one pass while all residuals are > 3e-6, CGS2 below */
-  int stencil_variant;   /* 0: marching kernel, rows per CTA chosen by level size (default); 1: shared-memory tiled kernel (reference
-                            implementation); 2: marching kernel with 32 rows per CTA on every level (round-1 behaviour); 3: like 0 without the wave-quantisation
-                            rule for the fine level */
   int mg_nu_growth;      /* extra Jacobi sweeps per coarser level (variable V-cycle), default 0 */
-  int use_graph;         /* 1 (default): replay the multigrid V-cycle as one CUDA graph (fp32 multigrid only) */
+  int use_graph;         /* 1 (default): replay the multigrid V-cycle as one CUDA graph */
   int mg_cycles;         /* V-cycles per preconditioner application (default 1) */
-  int mg_precision;      /* 1 (default): multigrid preconditioner in fp32 (Krylov iteration stays fp64); 0: all fp64 */
-  int inner_mode;        /* 1 (default): device-resident FGMRES cycles (fused Gram-Schmidt kernels, device least-squares, one or
-                            two host read-backs per cycle); 0: the round-1 host-driven FGMRES */
   int inner_ir;          /* 1 (default): run the FGMRES cycles in the multigrid precision (fp32) inside an fp64 iterative
-                            refinement (needs mg_precision == 1; diagonal path); 0: fp64 cycles */
+                            refinement (diagonal path); 0: fp64 cycles */
   double ir_floor;       /* smallest residual reduction asked of one fp32 cycle (default 1e-4) */
   double ir_trust;       /* solves whose tolerance is >= this accept the fp32 residual estimate without an fp64 check (3e-5) */
   double inner_relax_complex; /* complex-arithmetic problems: loosest inner tolerance = this x inner_tol (default 50) */
   int mg_fuse_first;     /* 1 (default): the first two pre-smoothing sweeps (from the zero guess) run as one kernel pass */
   int ks_keep;           /* Krylov-Schur: Ritz vectors kept at a restart; 0 (default) = k + (ncv - k) / 2 */
-  int transfer_tiled;    /* 1: shared-memory tiled restriction kernel on levels with >= 64 coarse columns (measured: no faster); 0 (default): per-thread gathers */
-  int warm_start;        /* 1: within one call, each device batch starts its Krylov spaces from the wanted Ritz vectors of the previous
-                            batch of the same shape (neighbouring frequencies of a sweep); 0 (default): seeded random start vector
-                            like the reference (solver.py:822-857) */
   double cluster_gap;    /* a wanted Ritz value closer than this (relative) to another Ritz value disables the relaxation of the inner
                             tolerance for that problem (default 1e-3) */
   int mg_fused_tail;     /* 1 (default): the multigrid levels that fit in shared memory together (<= 64^2 cells) run as one kernel, one
                             CTA per problem (csrc/coarse_kernel.cuh); 0: one kernel per operation on every level */
-  int stencil_async;     /* 1: stencil rows staged with cp.async (LDGSTS) into a shared-memory ring instead of prefetch registers (4/8-byte
-                            element types, no mu fields); 0: register-prefetch marching kernel */
   double kappa_cap;      /* the Ritz residual of a wanted pair is weighted by min(kappa, kappa_cap), kappa = condition number of the
                             Ritz value in the projected problem, before the comparison with eig_tol (default 1e4; 1 = ARPACK's test) */
   int outer_dgks;        /* 1 (default): Krylov-Schur orthogonalisation reorthogonalises only when ARPACK's DGKS test asks for it;
                             0: always two Gram-Schmidt passes */
-  int stencil_pair;      /* pair-marching stencil kernels for the real fp32 multigrid operators on even-width levels (two columns per thread,
-                            64-bit accesses, CTA width fitted to the row, six-fold unrolled row loop): 1 / 2 = rows prefetched into one / two
-                            sets of registers (csrc/march2.cuh); 3 / 4 = rows staged by TMA bulk copies (cp.async.bulk + mbarrier, ring of
-                            three stages, csrc/march2_tma.cuh) where ny % 4 == 0, the register version 1 / 2 elsewhere; 5 = TMA, two
-                            stages; 0 = the one-column marching kernel everywhere */
+  int stencil_pair;      /* 1 (default): pair-marching stencil kernels for the real fp32 multigrid operators on even-width levels (two columns
+                            per thread, 64-bit accesses, CTA width fitted to the row, six-fold unrolled row loop): rows staged by TMA bulk
+                            copies (cp.async.bulk + mbarrier, ring of three stages, csrc/march2_tma.cuh) where ny % 4 == 0 outside the fused
+                            first sweeps, prefetched into two sets of registers (csrc/march2.cuh) elsewhere; 0: the one-column marching
+                            kernel everywhere */
   int stencil_pair_rows; /* rows marched per CTA by the pair kernel (rounded to 6 m - 3); 0 (default) = chosen per level from the
                             number of resident CTAs */
   int transfer_vec;      /* multigrid transfers: bit 0 = the prolongation reads / writes its four fine values as one 128-bit access (fp32 vectors,

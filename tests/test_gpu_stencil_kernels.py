@@ -38,8 +38,8 @@ def test_pair_and_tma_kernels_match_the_one_column_kernel(shape, symmetry):
     sh = (C.c_int * 40)()
     n = _cabi.lib().b200ms_debug_hierarchy(C.byref(pk.struct), None, 20, sh)
     shapes = [(sh[2 * i], sh[2 * i + 1]) for i in range(n)]
-    hs = {sp: _cabi.Handle(stencil_pair=sp) for sp in (0, 1, 2, 4, 5)}
-    hs[9] = _cabi.Handle(stencil_pair=4, stencil_pair_rows=9)  # many short marches: every CTA boundary case
+    hs = {sp: _cabi.Handle(stencil_pair=sp) for sp in (0, 1)}
+    hs[9] = _cabi.Handle(stencil_pair=1, stencil_pair_rows=9)  # many short marches: every CTA boundary case
     rng = np.random.default_rng(7)
     try:
         for lvl, (nx, ny) in enumerate(shapes[:3]):
@@ -73,8 +73,7 @@ def test_vcycle_is_the_same_with_every_kernel_family(shape, symmetry):
         r[1][0, :] = 0
     ra = np.ascontiguousarray(r.ravel())
     zs = {}
-    for name, opts in (("round2", dict(stencil_pair=0, transfer_vec=0)), ("default", {}), ("pair_only", dict(stencil_pair=2, transfer_vec=0)),
-                       ("transfers_only", dict(stencil_pair=0, transfer_vec=3))):
+    for name, opts in (("round2", dict(stencil_pair=0, transfer_vec=0)), ("default", {}), ("transfers_only", dict(stencil_pair=0, transfer_vec=3))):
         h = _cabi.Handle(**opts)
         z = np.zeros(ra.size, complex)
         rc = _cabi.lib().b200ms_debug_vcycle(h._h, C.byref(pk.struct), _cabi._ptr(ra.view(float)), _cabi._ptr(z.view(float)))
@@ -84,5 +83,4 @@ def test_vcycle_is_the_same_with_every_kernel_family(shape, symmetry):
     scale = np.abs(zs["round2"]).max()
     assert np.isfinite(scale) and scale > 0
     assert np.abs(zs["transfers_only"] - zs["round2"]).max() <= 2e-6 * scale  # same expressions, same order
-    for name in ("default", "pair_only"):
-        assert np.abs(zs[name] - zs["round2"]).max() <= 2e-5 * scale, name
+    assert np.abs(zs["default"] - zs["round2"]).max() <= 2e-5 * scale

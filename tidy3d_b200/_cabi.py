@@ -17,7 +17,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B200MS_LIB") or os.path.join(_HERE, "libb200ms.so")  # B200MS_LIB: developer override (A/B of builds)
 
-ABI_VERSION = 203  # B200MS_VERSION of include/b200ms.h
+ABI_VERSION = 204  # B200MS_VERSION of include/b200ms.h
 OK, ERR_SHAPE, ERR_NO_MODES, ERR_UNSUPPORTED, ERR_CUDA, ERR_NOCONV, ERR_ARG = range(7)
 SPEC_NAMES = {0: "diagonal", 1: "tensorial_real", 2: "tensorial_complex"}
 
@@ -54,8 +54,8 @@ class Options(C.Structure):
         ("eig_tol", C.c_double), ("inner_tol", C.c_double), ("ncv", C.c_int), ("max_restarts", C.c_int),
         ("gmres_restart", C.c_int), ("gmres_maxit", C.c_int), ("mg_nu", C.c_int), ("mg_min_size", C.c_int),
         ("mg_coarse_iters", C.c_int), ("max_batch", C.c_int), ("mg_omega", C.c_double), ("mg_ppw", C.c_double),
-        ("verbose", C.c_int), ("mg_pml_phase", C.c_double), ("inner_relax", C.c_double), ("inner_relax_cap", C.c_double), ("gmres_cgs2", C.c_int), ("stencil_variant", C.c_int), ("mg_nu_growth", C.c_int), ("use_graph", C.c_int), ("mg_cycles", C.c_int), ("mg_precision", C.c_int),
-        ("inner_mode", C.c_int), ("inner_ir", C.c_int), ("ir_floor", C.c_double), ("ir_trust", C.c_double), ("inner_relax_complex", C.c_double), ("mg_fuse_first", C.c_int), ("ks_keep", C.c_int), ("transfer_tiled", C.c_int), ("warm_start", C.c_int), ("cluster_gap", C.c_double), ("mg_fused_tail", C.c_int), ("stencil_async", C.c_int), ("kappa_cap", C.c_double), ("outer_dgks", C.c_int), ("stencil_pair", C.c_int), ("stencil_pair_rows", C.c_int), ("transfer_vec", C.c_int), ("tensor_mg_cycles", C.c_int),
+        ("verbose", C.c_int), ("mg_pml_phase", C.c_double), ("inner_relax", C.c_double), ("inner_relax_cap", C.c_double), ("gmres_cgs2", C.c_int), ("mg_nu_growth", C.c_int), ("use_graph", C.c_int), ("mg_cycles", C.c_int),
+        ("inner_ir", C.c_int), ("ir_floor", C.c_double), ("ir_trust", C.c_double), ("inner_relax_complex", C.c_double), ("mg_fuse_first", C.c_int), ("ks_keep", C.c_int), ("cluster_gap", C.c_double), ("mg_fused_tail", C.c_int), ("kappa_cap", C.c_double), ("outer_dgks", C.c_int), ("stencil_pair", C.c_int), ("stencil_pair_rows", C.c_int), ("transfer_vec", C.c_int), ("tensor_mg_cycles", C.c_int),
     ]  # fmt: skip
 
 

@@ -60,11 +60,6 @@ struct b200ms_handle {
   DevBuf scan;        // reduction scratch + per-medium results of prepare_window
   DevBuf refs;        // MediumRef array of the batch being built
   DevBuf post;        // interpolation tables / partials / results of the on-device post-processing
-  DevBuf warm;        // sorted Ritz vectors of the previous device batch of this call ([k][B][len]): warm start of the next one
-  int warm_B = 0, warm_k = 0, warm_tsize = 0;
-  size_t warm_len = 0;
-  bool warm_valid = false;
-  long long warm_key[16];
   b200ms_options opt;
   std::string err;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -90,15 +85,12 @@ extern "C" void b200ms_default_options(b200ms_options *o) {
   o->mg_ppw = 4.0;
   o->verbose = 0;
   o->mg_pml_phase = 0.7853981633974483;
-  o->stencil_variant = 0;
-  o->mg_precision = 1;
   o->mg_cycles = 1;
   o->use_graph = 1;
   o->mg_nu_growth = 0;
   o->gmres_cgs2 = 2;
   o->inner_relax = 1.0;
   o->inner_relax_cap = 1e-4;
-  o->inner_mode = 1;
   o->inner_ir = 1;
   o->ir_floor = 1e-4;
   o->ir_trust = 3e-5;
@@ -106,13 +98,10 @@ extern "C" void b200ms_default_options(b200ms_options *o) {
   o->cluster_gap = 1e-3;
   o->mg_fuse_first = 1;
   o->ks_keep = 0;
-  o->transfer_tiled = 0;
-  o->warm_start = 0;
   o->mg_fused_tail = 1;
-  o->stencil_async = 0;
   o->kappa_cap = 1e4;
   o->outer_dgks = 1;
-  o->stencil_pair = 4;
+  o->stencil_pair = 1;
   o->stencil_pair_rows = 0;
   o->transfer_vec = 3;
   o->tensor_mg_cycles = 3;
@@ -152,7 +141,6 @@ extern "C" int b200ms_destroy(b200ms_handle *h) {
   h->scan.release();
   h->refs.release();
   h->post.release();
-  h->warm.release();
   if (h->io_stream) cudaStreamDestroy(h->io_stream);
   if (h->dl_stream) cudaStreamDestroy(h->dl_stream);
   if (h->flush_buf) cudaFree(h->flush_buf);
@@ -711,14 +699,7 @@ void solve_group(b200ms_handle *h, const std::vector<int> &ids, const Window &W,
     eig.nconv.assign(B, k);
     eig.resid.assign(B, 0.0);
   } else {
-    // consecutive device batches of one call are neighbouring slices of a sweep: start each problem's Krylov space from the
-    // wanted Ritz vectors of the problem at the same position of the previous batch (same group key, same shapes)
-    long long key[16] = {S.nx, S.ny, k, (long long)sizeof(T), S.tensor_ ? 1 : 0, S.has_mu ? 1 : 0, ps[0]->ax[0].pmc, ps[0]->ax[1].pmc,
-                         ps[0]->direction, ps[0]->masked ? 1 : 0, (long long)S.len, 0, 0, 0, 0, 0};
-    const bool warm = h->opt.warm_start && h->warm_valid && h->warm_B >= B && h->warm_k == k && h->warm_len == S.len &&
-                      h->warm_tsize == (int)sizeof(T) && std::memcmp(key, h->warm_key, sizeof(key)) == 0;
-    if (warm) S.init_start_from(reinterpret_cast<const T *>(h->warm.p), h->warm_B);
-    else S.init_start_vector(0);
+    S.init_start_vector(0);
     NvtxRange r("b200ms:eigen-iteration");
     eig = S.krylov_schur(real_arith);
   }
@@ -766,16 +747,6 @@ void solve_group(b200ms_handle *h, const std::vector<int> &ids, const Window &W,
       auto r = S.eigen_residuals(q, lq);
       for (int b = 0; b < B; ++b) maxres[b] = std::max(maxres[b], r[b]);
     }
-  }
-  if (h->opt.warm_start && !relative) {  // keep the sorted Ritz vectors for the next batch of this call
-    long long key[16] = {S.nx, S.ny, k, (long long)sizeof(T), S.tensor_ ? 1 : 0, S.has_mu ? 1 : 0, ps[0]->ax[0].pmc, ps[0]->ax[1].pmc,
-                         ps[0]->direction, ps[0]->masked ? 1 : 0, (long long)S.len, 0, 0, 0, 0, 0};
-    const size_t bytes = (size_t)k * S.vstride * sizeof(T);
-    h->warm.reserve(bytes + 256);
-    CUDA_CHECK(cudaMemcpyAsync(h->warm.p, S.ritz_ptr(), bytes, cudaMemcpyDeviceToDevice, h->stream));
-    std::memcpy(h->warm_key, key, sizeof(key));
-    h->warm_B = B; h->warm_k = k; h->warm_len = S.len; h->warm_tsize = (int)sizeof(T);
-    h->warm_valid = true;
   }
   CUDA_CHECK(cudaEventRecord(h->ev1, h->stream));
   CUDA_CHECK(cudaEventSynchronize(h->ev1));
@@ -837,20 +808,11 @@ size_t bytes_per_problem(const ProblemSetup &s, const b200ms_options &opt) {
 }
 
 template <typename... A>
-void dispatch_group(int kind, bool f32, A &&...a) {
+void dispatch_group(int kind, A &&...a) {
   switch (kind) {
-    case 0:
-      if (f32) solve_group<double, double, float, float>(std::forward<A>(a)...);
-      else solve_group<double, double, double, double>(std::forward<A>(a)...);
-      break;
-    case 1:
-      if (f32) solve_group<cplx, double, cplxf, float>(std::forward<A>(a)...);
-      else solve_group<cplx, double, cplx, double>(std::forward<A>(a)...);
-      break;
-    default:
-      if (f32) solve_group<cplx, cplx, cplxf, cplxf>(std::forward<A>(a)...);
-      else solve_group<cplx, cplx, cplx, cplx>(std::forward<A>(a)...);
-      break;
+    case 0: solve_group<double, double, float, float>(std::forward<A>(a)...); break;
+    case 1: solve_group<cplx, double, cplxf, float>(std::forward<A>(a)...); break;
+    default: solve_group<cplx, cplx, cplxf, cplxf>(std::forward<A>(a)...); break;
   }
 }
 
@@ -862,7 +824,6 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
   h->err.clear();
   std::memset(&h->stats, 0, sizeof(h->stats));
   h->stats.nprob = nprob;
-  h->warm_valid = false;  // warm starts never cross calls: a call's results depend on its own inputs only
   const auto call0 = std::chrono::steady_clock::now();
   int first_err = B200MS_OK;
   try {
@@ -940,7 +901,7 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
             unsigned char *region = ob.p + cursor;
             if (cursor + pb * ids.size() > ob.cap) throw std::runtime_error("output buffer accounting error");
             try {
-              dispatch_group(kv.first.kind, h->opt.mg_precision == 1, h, ids, W, prob, res, region, copies);
+              dispatch_group(kv.first.kind, h, ids, W, prob, res, region, copies);
             } catch (const DeviceOutOfMemory &) {
               // bytes_per_problem is an estimate (other processes, fragmentation): the arena is reserved before anything else
               // of the batch happens, so the same problems are simply solved in smaller device batches
@@ -1099,19 +1060,15 @@ extern "C" int b200ms_bench_stencil(b200ms_handle *h, const b200ms_problem *prob
       h->err = s.error;
       return s.status;
     }
-    const bool f32 = h->opt.mg_precision == 1;
     switch (kind_of(s)) {
       case 0:
-        if (f32) bench_group<double, double, float, float>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
-        else bench_group<double, double, double, double>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
+        bench_group<double, double, float, float>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
         break;
       case 1:
-        if (f32) bench_group<cplx, double, cplxf, float>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
-        else bench_group<cplx, double, cplx, double>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
+        bench_group<cplx, double, cplxf, float>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
         break;
       default:
-        if (f32) bench_group<cplx, cplx, cplxf, cplxf>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
-        else bench_group<cplx, cplx, cplx, cplx>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
+        bench_group<cplx, cplx, cplxf, cplxf>(h, W, nbatch, mode, nrep, flush_l2, x, y, ms_per_launch, bytes_per_apply);
         break;
     }
   } catch (const std::exception &e) {
@@ -1334,17 +1291,10 @@ int debug_dispatch(b200ms_handle *h, const b200ms_problem *prob, int what, int l
       h->err = s.error;
       return s.status;
     }
-    const bool f32 = h->opt.mg_precision == 1;
     switch (kind_of(s)) {
-      case 0:
-        return f32 ? debug_run<double, double, float, float>(h, W, what, level, mode, in0, in1, out, iters, relres)
-                   : debug_run<double, double, double, double>(h, W, what, level, mode, in0, in1, out, iters, relres);
-      case 1:
-        return f32 ? debug_run<cplx, double, cplxf, float>(h, W, what, level, mode, in0, in1, out, iters, relres)
-                   : debug_run<cplx, double, cplx, double>(h, W, what, level, mode, in0, in1, out, iters, relres);
-      default:
-        return f32 ? debug_run<cplx, cplx, cplxf, cplxf>(h, W, what, level, mode, in0, in1, out, iters, relres)
-                   : debug_run<cplx, cplx, cplx, cplx>(h, W, what, level, mode, in0, in1, out, iters, relres);
+      case 0: return debug_run<double, double, float, float>(h, W, what, level, mode, in0, in1, out, iters, relres);
+      case 1: return debug_run<cplx, double, cplxf, float>(h, W, what, level, mode, in0, in1, out, iters, relres);
+      default: return debug_run<cplx, cplx, cplxf, cplxf>(h, W, what, level, mode, in0, in1, out, iters, relres);
     }
   } catch (const std::exception &e) {
     h->err = e.what();

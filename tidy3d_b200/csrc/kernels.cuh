@@ -505,153 +505,6 @@ __global__ void __launch_bounds__(kMarchCols) stencil_march_kernel(StencilArgs<T
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// cp.async variant of the marching kernel (LDGSTS: asynchronous global -> shared copies, no staging registers).
-// Same march, same exchange of u / t through shared memory; what changes is how a thread gets its own column's row data:
-// instead of loading row k+3 into registers one step ahead (one global round trip per row step, the long-scoreboard stall
-// ncu shows for the register version), every thread keeps its next rows in flight as 4/8-byte cp.async copies into a
-// private four-slot ring in shared memory -- raw fields three row steps ahead, rhs / omega-over-diagonal one step ahead of
-// their use -- and waits with cp.async.wait_group.  No mu fields, no recomputed-diagonal mode (the multigrid hot path:
-// stored-diagonal sweep, residual, apply).
-// ------------------------------------------------------------------------------------------------
-template <int BYTES>
-__device__ __forceinline__ void cp_async_elem(void *smem, const void *gmem, bool valid) {
-  const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
-  const int src = valid ? BYTES : 0;  // src-size 0: the destination is zero-filled
-  asm volatile("cp.async.ca.shared.global [%0], [%1], %2, %3;\n" ::"r"(sa), "l"(gmem), "n"(BYTES), "r"(src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
-
-template <typename T, typename C, int MODE, int TXR>
-__global__ void __launch_bounds__(kMarchCols) stencil_march_async_kernel(StencilArgs<T, C> a) {
-  static_assert(MODE == MODE_APPLY || MODE == MODE_RESID || MODE == MODE_JACOBI_D, "cp.async variant: apply / residual / stored-diagonal sweep");
-  static_assert(sizeof(T) <= 8 && sizeof(C) <= 8, "cp.async.ca copies 4 or 8 bytes per element here");
-  constexpr int D = 4;  // ring depth (rows)
-  __shared__ T sB[2][kMarchCols + 2], sV[2][kMarchCols + 2], sU[2][kMarchCols + 2], sTt[2][kMarchCols + 2];
-  __shared__ T sX[4][TXR + 6];
-  __shared__ T rV1[D][kMarchCols], rV2[D][kMarchCols];
-  __shared__ C rEx[D][kMarchCols], rEy[D][kMarchCols], rIe[D][kMarchCols];
-  __shared__ T rR1[(MODE != MODE_APPLY) ? D : 1][kMarchCols], rR2[(MODE != MODE_APPLY) ? D : 1][kMarchCols];
-  __shared__ T rD1[(MODE == MODE_JACOBI_D) ? D : 1][kMarchCols], rD2[(MODE == MODE_JACOBI_D) ? D : 1][kMarchCols];
-
-  const int nx = a.nx, ny = a.ny;
-  const size_t N = (size_t)nx * ny;
-  const int b = blockIdx.z;
-  const int c = threadIdx.x;
-  const int gj = (int)blockIdx.x * kMarchOut - 1 + c;
-  const int i0 = blockIdx.y * TXR;
-  const int iend = (i0 + TXR < nx) ? i0 + TXR : nx;
-  const bool colv = (gj >= 0 && gj < ny);
-  const bool outc = colv && c >= 1 && c <= kMarchOut;
-  const T *x1 = a.x + (size_t)b * 2 * N, *x2 = x1 + N;
-  const C *fb = a.fields + a.field_bstride * b;
-  const C *exx = fb, *eyy = fb + N, *iez = fb + 2 * N;
-  const T *cx = a.cx + (size_t)b * 4 * nx, *cy = a.cy + (size_t)b * 4 * ny;
-  const T *r1 = (MODE != MODE_APPLY) ? a.rhs + (size_t)b * 2 * N : nullptr;
-  const T *dv = (MODE == MODE_JACOBI_D) ? a.dinv + (size_t)b * 2 * N : nullptr;
-  const T zT = zero_of<T>();
-
-  // one commit group per row step: raw row `gr` and rhs / dinv row `gq`
-  auto issue = [&](int gr, int gq) {
-    {
-      const bool v = colv && gr >= 0 && gr < nx && gr >= i0 - 1 && gr <= i0 + TXR;
-      const size_t g = v ? (size_t)gr * ny + gj : 0;
-      const int s = ((gr % D) + D) % D;
-      cp_async_elem<sizeof(T)>(&rV1[s][c], x1 + g, v);
-      cp_async_elem<sizeof(T)>(&rV2[s][c], x2 + g, v);
-      cp_async_elem<sizeof(C)>(&rEx[s][c], exx + g, v);
-      cp_async_elem<sizeof(C)>(&rEy[s][c], eyy + g, v);
-      cp_async_elem<sizeof(C)>(&rIe[s][c], iez + g, v);
-    }
-    if (MODE != MODE_APPLY) {
-      const bool v = outc && gq >= i0 && gq < iend;
-      const size_t g = v ? (size_t)gq * ny + gj : 0;
-      const int s = ((gq % D) + D) % D;
-      cp_async_elem<sizeof(T)>(&rR1[s][c], r1 + g, v);
-      cp_async_elem<sizeof(T)>(&rR2[s][c], r1 + N + g, v);
-      if (MODE == MODE_JACOBI_D) {
-        cp_async_elem<sizeof(T)>(&rD1[s][c], dv + g, v);
-        cp_async_elem<sizeof(T)>(&rD2[s][c], dv + N + g, v);
-      }
-    }
-    cp_async_commit();
-  };
-  // step `it` of the march issues raw row it+5 and rhs row it+3; the three steps before the loop are issue-only
-  issue(i0 - 1, i0 - 3);
-  issue(i0, i0 - 2);
-  issue(i0 + 1, i0 - 1);
-
-  for (int q = c; q < 4 * (TXR + 6); q += kMarchCols) {
-    const int w = q / (TXR + 6), r = q % (TXR + 6), gi = i0 - 3 + r;
-    sX[w][r] = (gi >= 0 && gi < nx) ? ldg(cx + (size_t)w * nx + gi) : zT;
-  }
-  for (int s = 0; s < 2; ++s) { sB[s][c + 1] = zT; sV[s][c + 1] = zT; sU[s][c + 1] = zT; sTt[s][c + 1] = zT; }
-  if (c < 2)
-    for (int s = 0; s < 2; ++s) {
-      const int e = c == 0 ? 0 : kMarchCols + 1;
-      sB[s][e] = zT; sV[s][e] = zT; sU[s][e] = zT; sTt[s][e] = zT;
-    }
-  T yf0 = zT, yf1 = zT, yb0 = zT, ybm = zT;
-  if (colv) { yf0 = ldg(cy + gj); yf1 = ldg(cy + ny + gj); yb0 = ldg(cy + 2 * ny + gj); ybm = ldg(cy + 3 * ny + gj); }
-  const T sg = ldg(a.sigma + b);
-  T *y1 = a.y + (size_t)b * 2 * N, *y2 = y1 + N;
-
-  T a1 = zT, b1 = zT, v11 = zT, v21 = zT, a0 = zT, b0 = zT, v10 = zT, v20 = zT;
-  C ie1 = C(), ie0 = C();
-  T u0 = zT, t0 = zT, tm = zT;
-  __syncthreads();
-
-  for (int k = i0 - 3; k < iend; ++k) {
-    const int s = k & 1, sp = s ^ 1;
-    const int xr = k - (i0 - 3);
-    cp_async_wait<2>();  // the group of step k-3 (raw row k+2, rhs row k) has landed; only this thread reads its ring entries
-    const int s2 = (((k + 2) % D) + D) % D, s0 = ((k % D) + D) % D;
-    const T v12 = rV1[s2][c], v22 = rV2[s2][c];
-    const C ex2 = rEx[s2][c], ey2 = rEy[s2][c], ie2 = rIe[s2][c];
-    T cr1 = zT, cr2 = zT, cd1 = zT, cd2 = zT;
-    if (MODE != MODE_APPLY) { cr1 = rR1[s0][c]; cr2 = rR2[s0][c]; }
-    if (MODE == MODE_JACOBI_D) { cd1 = rD1[s0][c]; cd2 = rD2[s0][c]; }
-    issue(k + 5, k + 3);  // slots of raw row k+1 and rhs row k-1, both consumed in the previous step
-    const T a2 = ex2 * v12, b2 = ey2 * v22;
-    // publish b[k+2], v1[k+2]
-    sB[s][c + 1] = b2;
-    sV[s][c + 1] = v12;
-    // u[k+1], t[k+1]
-    const T bl = sB[sp][c], v1r = sV[sp][c + 2];
-    const T xf0n = sX[0][xr + 1], xf1n = sX[1][xr + 1], xb0n = sX[2][xr + 1], xbmn = sX[3][xr + 1];
-    const T u1 = -(ie1 * (xb0n * a1 + xbmn * a0 + yb0 * b1 + ybm * bl));
-    const T t1 = xf0n * v21 + xf1n * v22 - yf0 * v11 - yf1 * v1r;
-    sU[s][c + 1] = u1;
-    sTt[s][c + 1] = t1;
-    // outputs of row k
-    if (outc && k >= i0) {
-      const T ur = sU[sp][c + 2], tl = sTt[sp][c];
-      const T xf0 = sX[0][xr], xf1 = sX[1][xr], xb0 = sX[2][xr], xbm = sX[3][xr];
-      T p1 = xf0 * u0 + xf1 * u1;
-      T p2 = yf0 * u0 + yf1 * ur;
-      p1 += yb0 * t0 + ybm * tl - a0;
-      p2 -= xb0 * t0 + xbm * tm + b0;
-      const T o1 = p1 - sg * v10, o2 = p2 - sg * v20;
-      const size_t g = (size_t)k * ny + gj;
-      if (MODE == MODE_APPLY) {
-        y1[g] = o1; y2[g] = o2;
-      } else if (MODE == MODE_RESID) {
-        y1[g] = cr1 - o1; y2[g] = cr2 - o2;
-      } else {
-        y1[g] = v10 + cd1 * (cr1 - o1); y2[g] = v20 + cd2 * (cr2 - o2);
-      }
-    }
-    tm = t0; t0 = t1; u0 = u1;
-    a0 = a1; b0 = b1; v10 = v11; v20 = v21; a1 = a2; b1 = b2; v11 = v12; v21 = v22;
-    ie0 = ie1; ie1 = ie2;
-    __syncthreads();
-  }
-  cp_async_wait<0>();
-  (void)ie0;
-}
-
 // y = omega * D^-1 rhs  (first Jacobi sweep from a zero guess; no halo needed)
 template <typename T, typename C, bool HAS_MU>
 __global__ void __launch_bounds__(256) jacobi0_kernel(StencilArgs<T, C> a) {
@@ -810,62 +663,6 @@ __global__ void __launch_bounds__(256) restrict4_kernel(TransferArgs a, const T 
   }
   if ((comp == 0 && a.mask_y && J == 0 && a.nyc > 1) || (comp == 1 && a.mask_x && I == 0 && a.nxc > 1)) acc = zero_of<T>();
   coarse[((size_t)b * 2 + comp) * Nc + (size_t)I * a.nyc + J] = acc;
-}
-
-// Shared-memory tiled restriction (element types of <= 8 bytes): a CTA produces an 8 x 64 tile of coarse values of one
-// component of one problem.  The fine window the tile depends on (<= 28 x 200 values for aggregates of <= 3 cells) is loaded
-// once with coalesced row reads; every coarse value is then a <= 4 x 4 weighted sum out of shared memory.  The per-thread
-// version above reads every fine value up to four times through L1 with stride-2 addresses and was the second largest
-// kernel of a V-cycle (162 us at 64 x 512^2 for 134 MB of input, profiles/r02_launch_shares.txt).
-constexpr int kRtI = 8, kRtJ = 64, kRtRows = 28, kRtCols = 200;
-template <typename T>
-__global__ void __launch_bounds__(256) restrict_tiled_kernel(TransferArgs a, const T *fine, T *coarse) {
-  __shared__ T tile[kRtRows][kRtCols];
-  __shared__ int win[4];
-  const int J0 = blockIdx.x * kRtJ, I0 = blockIdx.y * kRtI;
-  const int comp = blockIdx.z & 1, b = blockIdx.z >> 1;
-  const Transfer1DDev &tx = comp == 0 ? a.xe : a.xn;
-  const Transfer1DDev &ty = comp == 0 ? a.yn : a.ye;
-  const size_t Nf = (size_t)a.nxf * a.nyf, Nc = (size_t)a.nxc * a.nyc;
-  const T *f = fine + ((size_t)b * 2 + comp) * Nf;
-  const int tid = threadIdx.y * 64 + threadIdx.x;
-  const int I1 = min(I0 + kRtI, a.nxc), J1 = min(J0 + kRtJ, a.nyc);
-  if (tid == 0) {  // fine window of the tile (the lists are ascending in the fine index)
-    const int kx0 = tx.r_ptr[I0], kx1 = tx.r_ptr[I1], ky0 = ty.r_ptr[J0], ky1 = ty.r_ptr[J1];
-    win[0] = kx1 > kx0 ? tx.r_idx[kx0] : 0;
-    win[1] = kx1 > kx0 ? tx.r_idx[kx1 - 1] + 1 : 0;
-    win[2] = ky1 > ky0 ? ty.r_idx[ky0] : 0;
-    win[3] = ky1 > ky0 ? ty.r_idx[ky1 - 1] + 1 : 0;
-  }
-  __syncthreads();
-  const int r0 = win[0], nr = win[1] - win[0], c0 = win[2], nc = win[3] - win[2];
-  const bool fits = nr <= kRtRows && nc <= kRtCols;  // uniform over the CTA
-  if (fits) {
-    for (int e = tid; e < nr * nc; e += 256) {
-      const int r = e / nc, c = e % nc;
-      tile[r][c] = ldg(f + (size_t)(r0 + r) * a.nyf + c0 + c);
-    }
-  }
-  __syncthreads();
-  const int J = J0 + threadIdx.x;
-  for (int q = threadIdx.y; q < kRtI; q += 4) {
-    const int I = I0 + q;
-    if (I >= a.nxc || J >= a.nyc) continue;
-    T acc = zero_of<T>();
-    const int kx0 = tx.r_ptr[I], kx1 = tx.r_ptr[I + 1], ky0 = ty.r_ptr[J], ky1 = ty.r_ptr[J + 1];
-    for (int kx = kx0; kx < kx1; ++kx) {
-      const int fr = tx.r_idx[kx];
-      T racc = zero_of<T>();
-      if (fits) {
-        for (int ky = ky0; ky < ky1; ++ky) racc += ty.r_w[ky] * tile[fr - r0][ty.r_idx[ky] - c0];
-      } else {
-        for (int ky = ky0; ky < ky1; ++ky) racc += ty.r_w[ky] * ldg(f + (size_t)fr * a.nyf + ty.r_idx[ky]);
-      }
-      acc += tx.r_w[kx] * racc;
-    }
-    if ((comp == 0 && a.mask_y && J == 0 && a.nyc > 1) || (comp == 1 && a.mask_x && I == 0 && a.nxc > 1)) acc = zero_of<T>();
-    coarse[((size_t)b * 2 + comp) * Nc + (size_t)I * a.nyc + J] = acc;
-  }
 }
 
 // fine[b][comp] += P coarse[b][comp].  All index / weight loads and the four coarse loads are independent and issued

@@ -100,17 +100,16 @@ template <> inline cd to_cd<float>(float v) { return cd(v, 0.0); }
 template <> inline cd to_cd<cplxf>(cplxf v) { return cd(v.re, v.im); }
 
 // ------------------------------------------------------------------------------------------------------
-// T / C: Krylov vector and coefficient-field types (fp64).  P / PC: the same for the multigrid preconditioner,
-// either identical (all fp64) or their fp32 twins (mixed precision: the V-cycle moves half the bytes).
-template <typename T, typename C, typename P = T, typename PC = C>
+// T / C: Krylov vector and coefficient-field types (fp64).  P / PC: their fp32 twins, the types of the multigrid
+// preconditioner (mixed precision: the V-cycle moves half the bytes).
+template <typename T, typename C, typename P, typename PC>
 class BatchSolver {
  public:
-  static constexpr bool kMixed = !std::is_same<T, P>::value;
   struct Level {
     int nx = 0, ny = 0;
     size_t N = 0;
     PC *fields = nullptr;
-    C *fields_true = nullptr;  // level 0 only (aliases `fields` when PC == C)
+    C *fields_true = nullptr;  // level 0 only: fp64 fields of the reference operator
     size_t fbstride = 0;
     P *cx = nullptr, *cy = nullptr;          // multigrid (phase-limited PML) coefficients
     T *cx_true = nullptr, *cy_true = nullptr;  // level 0 only: the reference operator
@@ -156,7 +155,7 @@ class BatchSolver {
     m = std::min(ncv, (int)std::min<size_t>(len - 1, 1 << 20));
     if (m < k + 2) m = std::min<int>(k + 2, (int)len);
     restart = std::max(2, opt_.gmres_restart);
-    if (opt_.inner_mode != 0) restart = std::min(restart, kGsMaxCoef - 4);
+    restart = std::min(restart, kGsMaxCoef - 4);
     mask_x_ = (!p0.ax[0].pmc && nx > 1) ? 1 : 0;
     mask_y_ = (!p0.ax[1].pmc && ny > 1) ? 1 : 0;
 
@@ -182,7 +181,7 @@ class BatchSolver {
     const size_t fB = shared_fields ? 1 : B;
     for (int l = 0; l < L; ++l) {
       size_t Nl = (size_t)plan_.nx[l] * plan_.ny[l];
-      sz.add<C>(fB * nf * Nl * (l == 0 && kMixed ? 2 : 1));
+      sz.add<C>(fB * nf * Nl * (l == 0 ? 2 : 1));
       sz.add<T>((size_t)B * 4 * plan_.nx[l] * (l == 0 ? 2 : 1));
       sz.add<T>((size_t)B * 4 * plan_.ny[l] * (l == 0 ? 2 : 1));
       for (int q = 0; q < 5; ++q) sz.add<T>((size_t)B * 2 * Nl);
@@ -245,10 +244,7 @@ class BatchSolver {
       v.N = (size_t)v.nx * v.ny;
       v.fbstride = shared_fields ? 0 : nf * v.N;
       v.fields = arena_.get<PC>(fB * nf * v.N);
-      if (l == 0) {
-        if constexpr (kMixed) v.fields_true = arena_.get<C>(fB * nf * v.N);
-        else v.fields_true = reinterpret_cast<C *>(v.fields);
-      }
+      if (l == 0) v.fields_true = arena_.get<C>(fB * nf * v.N);
       v.cx = arena_.get<P>((size_t)B * 4 * v.nx);
       v.cy = arena_.get<P>((size_t)B * 4 * v.ny);
       if (l == 0) {
@@ -461,11 +457,11 @@ class BatchSolver {
     a.dinv = dinv;
     stats.launches++;
     if (launch_march2<TT, CC>(v, mode, a, dinv != nullptr)) return;
-    if (opt_.stencil_variant != 1 && v.nx >= 32 && v.ny >= 2) {
+    if (v.nx >= 32 && v.ny >= 2) {
       // rows marched per CTA: the march is a serial chain of (TXR + 3) row steps, each waiting on one global-load
       // round trip, so small levels (few CTAs per SM, nothing to hide that latency behind) get short chains
       bool rows32 = v.nx >= 384;
-      if (rows32 && opt_.stencil_variant != 2 && opt_.stencil_variant != 3) {
+      if (rows32) {
         // wave quantisation: 7 CTAs of 128 threads per SM are resident; when 32-row CTAs leave the last wave mostly empty
         // (e.g. 32 problems of 512^2: 2.47 waves) 16-row CTAs fill it at the price of 9 % more halo rows
         const double per_wave = 148.0 * 7.0;
@@ -474,7 +470,7 @@ class BatchSolver {
         const double t32 = std::ceil(c32) * 35.0, t16 = std::ceil(c16) * 19.0;  // waves x row steps per CTA
         if (t16 < 0.97 * t32) rows32 = false;
       }
-      if (rows32 || opt_.stencil_variant == 2) launch_march<TT, CC, 32>(v, mode, a, dinv != nullptr);
+      if (rows32) launch_march<TT, CC, 32>(v, mode, a, dinv != nullptr);
       else if (v.nx >= 192) launch_march<TT, CC, 16>(v, mode, a, dinv != nullptr);
       else launch_march<TT, CC, 8>(v, mode, a, dinv != nullptr);
       return;
@@ -491,55 +487,37 @@ class BatchSolver {
       else stencil_kernel<TT, CC, MODE_JACOBI, false><<<grd, blk, 0, st_>>>(a);
     }
   }
-  // pair-marching kernels (csrc/march2.cuh, csrc/march2_tma.cuh): real fp32 multigrid operators without mu fields on even-width
-  // levels.  stencil_pair: 1 / 2 = register version with one / two rows of prefetch registers; 3 / 4 = TMA row staging (ring of
-  // three stages) where it applies (ny % 4 == 0, not the fused first sweeps), register version 1 / 2 elsewhere; 5 = TMA with two stages.
+  // pair-marching kernels (csrc/march2.cuh, csrc/march2_tma.cuh), stencil_pair = 1: real fp32 multigrid operators without mu
+  // fields on even-width levels.  TMA row staging (ring of three stages) where it applies (ny % 4 == 0, not the fused first
+  // sweeps), the register version with two rows of prefetch registers elsewhere.
   using March2Fn = void (*)(StencilArgs<float, float>, int);
   struct March2Pick {
     March2Fn fn = nullptr;
-    int stages = 0, narr = 0, id = 0;  // stages > 0: TMA version with that ring depth
+    int stages = 0, narr = 0;  // stages > 0: TMA version with that ring depth
   };
   March2Pick march2_pick(int md, int ny) const {
     March2Pick p;
-    const int sp = opt_.stencil_pair;
-    const int pf = (sp == 2 || sp == 4) ? 2 : 1;
-    const int stages = (sp == 3 || sp == 4) ? 3 : (sp == 5 ? 2 : 0);
-    if (stages > 0 && (ny % 4) == 0 && md != MODE_JACOBI_D0) {
-      p.stages = stages;
+    if ((ny % 4) == 0 && md != MODE_JACOBI_D0) {
+      p.stages = 3;
       p.narr = md == MODE_APPLY ? 5 : (md == MODE_RESID ? 7 : 9);
-      p.id = 16 + stages;
-      if (stages == 3) {
-        if (md == MODE_APPLY) p.fn = stencil_march2_tma_kernel<MODE_APPLY, 3>;
-        else if (md == MODE_RESID) p.fn = stencil_march2_tma_kernel<MODE_RESID, 3>;
-        else if (md == MODE_JACOBI_D) p.fn = stencil_march2_tma_kernel<MODE_JACOBI_D, 3>;
-      } else {
-        if (md == MODE_APPLY) p.fn = stencil_march2_tma_kernel<MODE_APPLY, 2>;
-        else if (md == MODE_RESID) p.fn = stencil_march2_tma_kernel<MODE_RESID, 2>;
-        else if (md == MODE_JACOBI_D) p.fn = stencil_march2_tma_kernel<MODE_JACOBI_D, 2>;
-      }
+      if (md == MODE_APPLY) p.fn = stencil_march2_tma_kernel<MODE_APPLY, 3>;
+      else if (md == MODE_RESID) p.fn = stencil_march2_tma_kernel<MODE_RESID, 3>;
+      else if (md == MODE_JACOBI_D) p.fn = stencil_march2_tma_kernel<MODE_JACOBI_D, 3>;
       return p;
     }
-    p.id = pf;
-    if (pf == 1) {
-      if (md == MODE_APPLY) p.fn = stencil_march2_kernel<float, MODE_APPLY, 1>;
-      else if (md == MODE_RESID) p.fn = stencil_march2_kernel<float, MODE_RESID, 1>;
-      else if (md == MODE_JACOBI_D) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D, 1>;
-      else if (md == MODE_JACOBI_D0) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D0, 1>;
-    } else {
-      if (md == MODE_APPLY) p.fn = stencil_march2_kernel<float, MODE_APPLY, 2>;
-      else if (md == MODE_RESID) p.fn = stencil_march2_kernel<float, MODE_RESID, 2>;
-      else if (md == MODE_JACOBI_D) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D, 2>;
-      else if (md == MODE_JACOBI_D0) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D0, 2>;
-    }
+    if (md == MODE_APPLY) p.fn = stencil_march2_kernel<float, MODE_APPLY, 2>;
+    else if (md == MODE_RESID) p.fn = stencil_march2_kernel<float, MODE_RESID, 2>;
+    else if (md == MODE_JACOBI_D) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D, 2>;
+    else if (md == MODE_JACOBI_D0) p.fn = stencil_march2_kernel<float, MODE_JACOBI_D0, 2>;
     return p;
   }
   bool march2_eligible(const Level &v) const {
-    return opt_.stencil_pair > 0 && opt_.stencil_variant != 1 && !has_mu && !(v.ny & 1) && v.ny >= 8 && v.nx >= 32;
+    return opt_.stencil_pair > 0 && !has_mu && !(v.ny & 1) && v.ny >= 8 && v.nx >= 32;
   }
   static size_t march2_smem(const March2Pick &p, int W) { return (size_t)p.stages * p.narr * W * sizeof(float2); }
   // resident CTAs on the device for this kernel at this CTA width; also raises the kernel's dynamic shared-memory limit once
   int march2_resident(const March2Pick &p, int md, int W) {
-    const long key = ((long)md * 32 + p.id) * 1024 + W;
+    const long key = ((long)md * 32 + p.stages) * 1024 + W;
     auto it = m2_resident_.find(key);
     if (it == m2_resident_.end()) {
       int per_sm = 0, dev = 0, sms = 148;
@@ -592,15 +570,6 @@ class BatchSolver {
   template <typename TT, typename CC, int TXR>
   void launch_march(const Level &v, int mode, const StencilArgs<TT, CC> &a, bool have_dinv) {
     dim3 blk(kMarchCols), grd((v.ny + kMarchOut - 1) / kMarchOut, (v.nx + TXR - 1) / TXR, B);
-    if constexpr (sizeof(TT) <= 8 && sizeof(CC) <= 8) {
-      // cp.async (LDGSTS) variant: the multigrid hot path -- stored-diagonal sweep, residual, apply -- without mu fields
-      if (opt_.stencil_async && !has_mu && mode != MODE_JACOBI_D0 && (mode != MODE_JACOBI || have_dinv)) {
-        if (mode == MODE_JACOBI) stencil_march_async_kernel<TT, CC, MODE_JACOBI_D, TXR><<<grd, blk, 0, st_>>>(a);
-        else if (mode == MODE_RESID) stencil_march_async_kernel<TT, CC, MODE_RESID, TXR><<<grd, blk, 0, st_>>>(a);
-        else stencil_march_async_kernel<TT, CC, MODE_APPLY, TXR><<<grd, blk, 0, st_>>>(a);
-        return;
-      }
-    }
     if (mode == MODE_JACOBI_D0) {  // two sweeps from zero in one pass (needs the stored diagonal)
       if (has_mu) stencil_march_kernel<TT, CC, MODE_JACOBI_D0, true, TXR><<<grd, blk, 0, st_>>>(a);
       else stencil_march_kernel<TT, CC, MODE_JACOBI_D0, false, TXR><<<grd, blk, 0, st_>>>(a);
@@ -721,28 +690,17 @@ class BatchSolver {
   void precondition_E(const T *v, size_t v_bs, T *z, size_t z_bs) {
     const int ncyc = mg_cycles_();
     dim3 cg((unsigned)std::min<size_t>((lenE + 255) / 256, 1024), B);
-    if constexpr (kMixed) {
-      convert_strided_kernel<T, P><<<cg, 256, 0, st_>>>(lenE, v, v_bs, lv[0].b, lenE);
-      if (graph_exec_) {
-        CUDA_CHECK(cudaGraphLaunch(graph_exec_, st_));
-        stats.launches += graph_nodes_;
-        stats.stencil_applies += graph_fine_applies_;
-      } else {
-        precondition_body(lv[0].b, nullptr, ncyc);
-        graph_result_ = ncyc == 1 ? lv[0].x : pre_b_;
-      }
-      convert_strided_kernel<P, T><<<cg, 256, 0, st_>>>(lenE, graph_result_, lenE, z, z_bs);
-      stats.launches += 2;
+    convert_strided_kernel<T, P><<<cg, 256, 0, st_>>>(lenE, v, v_bs, lv[0].b, lenE);
+    if (graph_exec_) {
+      CUDA_CHECK(cudaGraphLaunch(graph_exec_, st_));
+      stats.launches += graph_nodes_;
+      stats.stencil_applies += graph_fine_applies_;
     } else {
-      if (v_bs == lenE && z_bs == lenE) {
-        precondition_body(v, z, ncyc);
-      } else {
-        convert_strided_kernel<T, P><<<cg, 256, 0, st_>>>(lenE, v, v_bs, lv[0].b, lenE);
-        precondition_body(lv[0].b, pre_b_, ncyc);
-        convert_strided_kernel<P, T><<<cg, 256, 0, st_>>>(lenE, pre_b_, lenE, z, z_bs);
-        stats.launches += 2;
-      }
+      precondition_body(lv[0].b, nullptr, ncyc);
+      graph_result_ = ncyc == 1 ? lv[0].x : pre_b_;
     }
+    convert_strided_kernel<P, T><<<cg, 256, 0, st_>>>(lenE, graph_result_, lenE, z, z_bs);
+    stats.launches += 2;
   }
   // V-cycles per application of the E-block inverse.  The tensorial block preconditioner needs an accurate one: its H block is
   // -(1/s)(I - Q B_E P), the difference of two O(K^2) terms (K = 1/(k0 h)) whose exact value is O(K^-2), so a B_E with the ~0.15
@@ -766,34 +724,32 @@ class BatchSolver {
       stats.launches++;
     }
   }
-  // Capture the V-cycle(s) into a CUDA graph (mixed precision only: its input and output buffers are fixed).  The
-  // cycle is ~60-250 small launches; replaying it as one graph removes most of the launch latency of the coarse levels.
+  // Capture the V-cycle(s) into a CUDA graph (its input and output buffers are fixed).  The cycle is ~60-250 small
+  // launches; replaying it as one graph removes most of the launch latency of the coarse levels.
   void capture_precondition_graph() {
-    if constexpr (kMixed) {
-      if (!opt_.use_graph) return;
-      const int ncyc = mg_cycles_();
-      const long l0 = stats.launches, a0 = stats.stencil_applies;
-      cudaGraph_t graph = nullptr;
-      CUDA_CHECK(cudaStreamSynchronize(st_));
-      CUDA_CHECK(cudaStreamBeginCapture(st_, cudaStreamCaptureModeRelaxed));
-      precondition_body(lv[0].b, nullptr, ncyc);
-      cudaError_t e = cudaStreamEndCapture(st_, &graph);
-      graph_nodes_ = stats.launches - l0;
-      graph_fine_applies_ = stats.stencil_applies - a0;
-      stats.launches = l0;
-      stats.stencil_applies = a0;
-      graph_result_ = ncyc == 1 ? lv[0].x : pre_b_;
-      if (e != cudaSuccess || !graph) {
-        cudaGetLastError();
-        graph_exec_ = nullptr;
-        return;
-      }
-      if (cudaGraphInstantiate(&graph_exec_, graph, 0) != cudaSuccess) {
-        cudaGetLastError();
-        graph_exec_ = nullptr;
-      }
-      cudaGraphDestroy(graph);
+    if (!opt_.use_graph) return;
+    const int ncyc = mg_cycles_();
+    const long l0 = stats.launches, a0 = stats.stencil_applies;
+    cudaGraph_t graph = nullptr;
+    CUDA_CHECK(cudaStreamSynchronize(st_));
+    CUDA_CHECK(cudaStreamBeginCapture(st_, cudaStreamCaptureModeRelaxed));
+    precondition_body(lv[0].b, nullptr, ncyc);
+    cudaError_t e = cudaStreamEndCapture(st_, &graph);
+    graph_nodes_ = stats.launches - l0;
+    graph_fine_applies_ = stats.stencil_applies - a0;
+    stats.launches = l0;
+    stats.stencil_applies = a0;
+    graph_result_ = ncyc == 1 ? lv[0].x : pre_b_;
+    if (e != cudaSuccess || !graph) {
+      cudaGetLastError();
+      graph_exec_ = nullptr;
+      return;
     }
+    if (cudaGraphInstantiate(&graph_exec_, graph, 0) != cudaSuccess) {
+      cudaGetLastError();
+      graph_exec_ = nullptr;
+    }
+    cudaGraphDestroy(graph);
   }
   ~BatchSolver() {
     if (graph_exec_) cudaGraphExecDestroy(graph_exec_);
@@ -865,7 +821,7 @@ class BatchSolver {
       return;
     }
     // (real fp32 only: the complex variant needs more registers and measured 3 % slower on c3_512)
-    if (nu >= 2 && dinv_ready_ && opt_.mg_fuse_first && sizeof(P) <= 4 && opt_.stencil_variant != 1 && v.nx >= 32 && v.ny >= 2) {
+    if (nu >= 2 && dinv_ready_ && opt_.mg_fuse_first && sizeof(P) <= 4 && v.nx >= 32 && v.ny >= 2) {
       apply(l, MODE_JACOBI_D0, cur, rin, cur);  // sweeps 1 and 2 from the zero guess in one pass (x argument unused)
       for (int s = 2; s < nu; ++s) {
         sweep(oth);
@@ -881,27 +837,16 @@ class BatchSolver {
     apply(l, MODE_RESID, cur, rin, v.r);
     {
       const TransferArgs &t = v.tr;
-      dim3 blk(64, 4);
-      if constexpr (sizeof(P) <= 8) {
-        if (opt_.transfer_tiled && t.nyc >= 64) {
-          dim3 grd((t.nyc + kRtJ - 1) / kRtJ, (t.nxc + kRtI - 1) / kRtI, 2 * B);
-          restrict_tiled_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
-        } else {
-          dim3 grd((t.nyc + 63) / 64, (t.nxc + 3) / 4, 2 * B);
-          const bool packed = (opt_.transfer_vec & 2) && std::is_same<typename RealOf<P>::type, float>::value && t.xn.r4 && t.xe.r4 && t.yn.r4 && t.ye.r4;
-          if (packed) restrict4_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
-          else restrict_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
-        }
-      } else {
-        dim3 grd((t.nyc + 63) / 64, (t.nxc + 3) / 4, 2 * B);
-        restrict_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
-      }
+      dim3 blk(64, 4), grd((t.nyc + 63) / 64, (t.nxc + 3) / 4, 2 * B);
+      const bool packed = (opt_.transfer_vec & 2) && t.xn.r4 && t.xe.r4 && t.yn.r4 && t.ye.r4;
+      if (packed) restrict4_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
+      else restrict_kernel<P><<<grd, blk, 0, st_>>>(t, v.r, lv[l + 1].b);
       stats.launches += 2;
     }
     vcycle(l + 1, lv[l + 1].b, nullptr);
     {
       const TransferArgs &t = v.tr;
-      if (t.nyf >= 256 && opt_.transfer_tiled != 2) {  // four fine columns per thread
+      if (t.nyf >= 256) {  // four fine columns per thread
         dim3 blk(64, 4), grd((t.nyf + 255) / 256, (t.nxf + 3) / 4, 2 * B);
         if ((opt_.transfer_vec & 1) && std::is_same<P, float>::value && (t.nyf % 4) == 0) prolong_add4_kernel<P, true><<<grd, blk, 0, st_>>>(t, lv[l + 1].x, cur);
         else prolong_add4_kernel<P, false><<<grd, blk, 0, st_>>>(t, lv[l + 1].x, cur);
@@ -1299,7 +1244,7 @@ class BatchSolver {
     U *Vu = reinterpret_cast<U *>(Vg_), *Zu = reinterpret_cast<U *>(Zg_), *Hu = reinterpret_cast<U *>(Hd_);
     U *yu = reinterpret_cast<U *>(ydev_);
     const int ld = restart + 4;
-    constexpr bool kStage = kMixed && std::is_same<U, P>::value;
+    constexpr bool kStage = std::is_same<U, P>::value;
     CUDA_CHECK(cudaMemcpyAsync(tol_dev_, tol.data(), B * sizeof(double), cudaMemcpyHostToDevice, st_));
     double tmin = 1.0;
     for (int b = 0; b < B; ++b)
@@ -1353,9 +1298,9 @@ class BatchSolver {
   double solve_op(const T *rhs, T *xsol, int &iters_out, const std::vector<char> *skip = nullptr, const std::vector<double> *tolv = nullptr) {
     // the tensorial path stays on the round-1 host-driven fp64 FGMRES: with no fp32 cycles to gain from, its adaptive
     // one-pass Gram-Schmidt is ~10 % faster than always-CGS2 device cycles (angled_64: 2 109 vs 2 322 ms)
-    if (opt_.inner_mode == 0 || tensor_) return fgmres(rhs, xsol, iters_out, skip, tolv);
+    if (tensor_) return fgmres(rhs, xsol, iters_out, skip, tolv);
     auto tol_of = [&](int b) { return tolv ? (*tolv)[b] : opt_.inner_tol; };
-    bool ir = kMixed && !tensor_ && !masked_ && opt_.inner_ir != 0;  // the fp32 twin of the operator keeps the PEC model: no masking
+    bool ir = !masked_ && opt_.inner_ir != 0;  // the fp32 twin of the operator keeps the PEC model: no masking
     std::vector<char> done(B, 0);
     if (skip) done = *skip;
     std::vector<unsigned char> hskip(B);
@@ -1495,25 +1440,6 @@ class BatchSolver {
     scale_inv_norm(rhs_, Vout_, hbuf_, hstride());
   }
 
-  // Start vector = normalised sum of the k Ritz vectors of another batch of the same shape (device, [k][Bw][len]): the
-  // Krylov space starts inside the wanted invariant subspace of a neighbouring frequency instead of at a random vector.
-  void init_start_from(const T *warm, int Bw) {
-    std::vector<T> ones((size_t)B * k, from_real<T>(1.0));
-    CUDA_CHECK(cudaMemcpyAsync(qbuf_, ones.data(), ones.size() * sizeof(T), cudaMemcpyHostToDevice, st_));
-    if (Bw == B) {
-      dim3 grd(vec_blocks(), B);
-      lincomb_kernel<T><<<grd, 256, (size_t)k * sizeof(T), st_>>>(warm, vstride, len, qbuf_, k, 1, 1, rhs_, vstride);
-    } else {  // a shorter last window: problem b starts from problem b of the previous window (Bw >= B)
-      dim3 grd(vec_blocks(), B);
-      lincomb_kernel<T><<<grd, 256, (size_t)k * sizeof(T), st_>>>(warm, (size_t)Bw * len, len, qbuf_, k, 1, 1, rhs_, vstride);
-    }
-    stats.launches++;
-    if (!tensor_) mask_E(rhs_, len);
-    dots(rhs_, 1, rhs_, hbuf_, hstride(), 0, false);
-    scale_inv_norm(rhs_, Vout_, hbuf_, hstride());
-    CUDA_CHECK(cudaStreamSynchronize(st_));
-  }
-
   EigResult krylov_schur(bool real_arith) {
     EigResult out;
     out.theta.assign((size_t)B * k, cd(0, 0));
@@ -1536,7 +1462,7 @@ class BatchSolver {
         double worst = solve_op(vj, w, its, &done, &tolv);
         stats.op_applies++;
         if (!(worst <= 1e-3)) stats.inner_failures++;
-        if (opt_.inner_mode != 0 && j + 2 < kGsMaxCoef) orthonormalise_dev(Vout_, j + 1, w, w, h, nrm, &done);
+        if (j + 2 < kGsMaxCoef) orthonormalise_dev(Vout_, j + 1, w, w, h, nrm, &done);
         else orthonormalise(Vout_, j + 1, w, w, h, nrm);
         for (int b = 0; b < B; ++b) {
           if (done[b]) continue;
@@ -1969,7 +1895,7 @@ class BatchSolver {
   cplx *tcoef_ = nullptr;
   std::vector<cd> sig_mg_host_;
   bool dinv_ready_ = false;
-  std::map<long, int> m2_resident_;  // pair-marching kernel: resident CTAs on the device per (mode, prefetch depth, CTA width)
+  std::map<long, int> m2_resident_;  // pair-marching kernel: resident CTAs on the device per (mode, TMA or registers, CTA width)
   cudaGraphExec_t graph_exec_ = nullptr;
   P *graph_result_ = nullptr;
   long graph_nodes_ = 0, graph_fine_applies_ = 0;

@@ -115,10 +115,6 @@ def full(names):
 
 if __name__ == "__main__":
     which = sys.argv[1:] or ["comp", "full"]
-    if "tiled" in which:
-        H.set_options(stencil_variant=1)
-    if "f64" in which:
-        H.set_options(mg_precision=0)
     if "comp" in which:
         for name in ["c1_64", "c1_64_sym_pmc_pec", "c3_96", "lossy_48", "c4_96", "nonuniform_56", "slab1d_x1", "slab1d_y1", "strip_128_m4", "c4_128"]:
             fac, kw, _ = CASES[name]
