@@ -13,7 +13,8 @@
  *   b200ms_problem       <->  the argument list above; mode_spec fields as read at
  *                             solver.py:86-90,198,204,247 (tidy3d/components/mode.py:18-209).
  *   b200ms_result        <->  the returned tuple (fields[2,3,Nx,Ny,1,M], n_complex[M], eps_spec)
- *                             (solver.py:257-269).
+ *                             (solver.py:257-269), plus what the reference does not return: on-device
+ *                             post-processing results and the permittivity gradient dn/deps (grad_eps).
  *   error codes          <->  ValueError / RuntimeError raised at solver.py:107, 876, 901.
  *
  * Plain C types only (no torch, no C++).  Host pointers in and out; the library owns all device
@@ -29,7 +30,7 @@
 extern "C" {
 #endif
 
-#define B200MS_VERSION 204
+#define B200MS_VERSION 205
 
 /* return codes */
 enum {
@@ -165,6 +166,13 @@ typedef struct {
                             was in, operator data already resident in HBM, results still on the device */
   double total_ms;       /* out: host wall time of that batch incl. upload of the operator and download of the fields */
   double max_residual;   /* out: max_i ||A v_i - lambda_i v_i|| / (|lambda_i| ||v_i||) */
+  /* ---- since version 205 ---- */
+  double *grad_eps;      /* NULL, or caller-allocated num_modes*3*nx*ny complex128 (re,im), HOST or DEVICE memory like `fields`:
+                            d n_complex[m] / d eps_cc[ix][iy] for c = xx, yy, zz, layout [mode][c][ix][iy] (y fastest), from the
+                            left eigenvector of the diagonal operator (DESIGN.md section 10; no extra solve, works without
+                            `fields`).  Diagonal problems only: a problem that asks for it and is tensorial / angled, bent, has
+                            mu / split_curl_scaling (incidence), basis fields or PEC-valued cells gets status
+                            B200MS_ERR_UNSUPPORTED before it is solved; the other problems of the call are unaffected */
 } b200ms_result;
 
 /* Tunables (all have defaults; see DESIGN.md). */
@@ -257,7 +265,8 @@ int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_problem *prob, 
  * of the operator of `prob` and return the mean kernel time (CUDA events on the library stream).
  * mode 0: y = (A - sigma) x, the fp64 operator apply of the Krylov iteration; mode 1: the production smoother sweep
  * (stored-diagonal Jacobi in the multigrid precision); mode 2: one fused CGS2 Gram-Schmidt step of the inner solver against
- * four basis vectors in the multigrid precision (gs_dots, gs_update_dots, gs_update_norm, gs_scale: 19 vector passes).  x (2*nx*ny complex128 (re,im)) may be NULL (random); y may be
+ * four basis vectors in the multigrid precision (gs_dots, gs_update_dots, gs_update_norm, gs_scale: 19 vector passes); mode 3: the two
+ * permittivity-gradient kernels (csrc/sensitivity.cuh) for prob.num_modes modes, N*M*(2*(2*s_v + 3*s_c) + 48) bytes per problem.  x (2*nx*ny complex128 (re,im)) may be NULL (random); y may be
  * NULL.  bytes_per_apply returns the algorithmic bytes of one launch (SURVEY 8(d)): N*(4*s_v + nf*s_c) per problem for
  * the apply, N*(8*s_v + nf*s_c) for the sweep. */
 int b200ms_bench_stencil(b200ms_handle *h, const b200ms_problem *prob, int nbatch, int mode, int nrep,
@@ -272,6 +281,10 @@ int b200ms_debug_schur(int n, const double *a, double *t, double *q);
  * (f0,f1,b0,bm complex) and fields[6*nx*ny] complex (exx,eyy,ezz,mxx,myy,mzz). NULL outputs skipped. */
 int b200ms_debug_setup(const b200ms_problem *prob, double *sigma, int *flags, double *target,
                        double *knorm, double *coef_x, double *coef_y, double *fields);
+/* the permittivity gradient of one mode of `prob` from a given eigenvector, by the functions the device kernel calls
+ * (csrc/sensitivity.cuh): vec = 2*nx*ny complex (re,im) [Ex|Ey] in solver units, lambda = its eigenvalue (re,im) of A = P Q
+ * (-n^2), out = 3*nx*ny complex (re,im) dn/deps_{xx,yy,zz}.  B200MS_ERR_UNSUPPORTED outside the scope of grad_eps */
+int b200ms_debug_sensitivity(const b200ms_problem *prob, const double *vec, const double *lambda, double *out);
 /* multigrid hierarchy shapes for a problem: writes up to max_levels (nx,ny) pairs, returns count */
 int b200ms_debug_hierarchy(const b200ms_problem *prob, const b200ms_options *opt, int max_levels,
                            int *shapes);

@@ -17,7 +17,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B200MS_LIB") or os.path.join(_HERE, "libb200ms.so")  # B200MS_LIB: developer override (A/B of builds)
 
-ABI_VERSION = 204  # B200MS_VERSION of include/b200ms.h
+ABI_VERSION = 205  # B200MS_VERSION of include/b200ms.h
 OK, ERR_SHAPE, ERR_NO_MODES, ERR_UNSUPPORTED, ERR_CUDA, ERR_NOCONV, ERR_ARG = range(7)
 SPEC_NAMES = {0: "diagonal", 1: "tensorial_real", 2: "tensorial_complex"}
 
@@ -46,6 +46,7 @@ class Result(C.Structure):
         ("fields", _dp), ("n_complex", _dp), ("flux", _dp), ("te_fraction", _dp), ("overlap_prev", _dp), ("eps_spec", C.c_int), ("status", C.c_int), ("converged", C.c_int),
         ("outer_iters", C.c_int), ("op_applies", C.c_int), ("inner_iters", C.c_int), ("stencil_applies", C.c_int),
         ("is_complex", C.c_int), ("solve_ms", C.c_double), ("total_ms", C.c_double), ("max_residual", C.c_double),
+        ("grad_eps", _dp),
     ]  # fmt: skip
 
 
@@ -71,6 +72,7 @@ EXPORTS = [
     "b200ms_version", "b200ms_get_stats", "b200ms_default_options", "b200ms_create", "b200ms_destroy", "b200ms_set_options",
     "b200ms_last_error", "b200ms_host_alloc", "b200ms_host_free", "b200ms_solve_batch", "b200ms_bench_stencil", "b200ms_debug_schur", "b200ms_debug_setup",
     "b200ms_debug_hierarchy", "b200ms_debug_apply", "b200ms_debug_vcycle", "b200ms_debug_solve", "b200ms_debug_march2_geometry", "b200ms_debug_post_tables", "b200ms_debug_post_tables_bounded", "b200ms_debug_te_terms", "b200ms_debug_grid_factors",
+    "b200ms_debug_sensitivity",
 ]  # fmt: skip
 
 _lib = None
@@ -119,6 +121,7 @@ def lib():
             L.b200ms_debug_post_tables_bounded.argtypes = [_dp, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, _ip, _dp, _dp]
             L.b200ms_debug_te_terms.argtypes = [_dp, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, _dp]
             L.b200ms_debug_grid_factors.argtypes = [C.POINTER(Problem), _dp, _dp, _dp]
+            L.b200ms_debug_sensitivity.argtypes = [C.POINTER(Problem), _dp, _dp, _dp]
             _lib = L
     return _lib
 
@@ -314,18 +317,32 @@ class Handle:
         except Exception:
             pass
 
-    def solve_batch(self, packed, want_fields=True, fields_ptrs=None, want_flux=False, want_overlaps=False):
+    def solve_batch(self, packed, want_fields=True, fields_ptrs=None, want_flux=False, want_overlaps=False, grad_eps=None,
+                    grad_eps_ptrs=None):
         """packed: list of PackedProblem.  Returns (rc, fields list | None, n_complex list, Result structs).
 
         ``fields_ptrs``: optional list of raw addresses (host or DEVICE memory, e.g. ``tensor.data_ptr()``) the library
         writes the fields of each problem to, instead of freshly allocated pinned host arrays; then ``fields`` is None.
-        Fields are complex128, or complex64 for ``precision == "single"`` problems (solver.py:265-267)."""
+        Fields are complex128, or complex64 for ``precision == "single"`` problems (solver.py:265-267).
+
+        ``grad_eps``: optional list of bools, one per problem: allocate a (M, 3, Nx, Ny) complex128 array for dn/deps of that
+        problem (``self.last_grad``, None where not asked).  ``grad_eps_ptrs``: list of raw addresses (host or device, 0 = none)
+        the library writes the gradient to instead."""
         n = len(packed)
         probs = (Problem * n)(*[p.struct for p in packed])
         results = (Result * n)()
         fields, ncs = [], []
-        self.last_flux, self.last_te, self.last_overlaps = [], [], []
+        self.last_flux, self.last_te, self.last_overlaps, self.last_grad = [], [], [], []
         for i, p in enumerate(packed):
+            if grad_eps_ptrs is not None:
+                results[i].grad_eps = C.cast(C.c_void_p(int(grad_eps_ptrs[i])), _dp) if grad_eps_ptrs[i] else None
+                self.last_grad.append(None)
+            elif grad_eps is not None and grad_eps[i]:
+                g = np.zeros((p.num_modes, 3, p.nx, p.ny), dtype=np.complex128)
+                self.last_grad.append(g)
+                results[i].grad_eps = _ptr(g.view(np.float64))
+            else:
+                self.last_grad.append(None)
             nc = np.zeros(p.num_modes, dtype=np.complex128)
             ncs.append(nc)
             results[i].n_complex = _ptr(nc.view(np.float64))

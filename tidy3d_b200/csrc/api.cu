@@ -661,9 +661,19 @@ struct FieldCopy {  // one pending delivery of packed fields: device region -> c
   size_t bytes;
 };
 
+// Why the permittivity gradient (b200ms_result.grad_eps) is not available for a problem; nullptr when it is (csrc/sensitivity.cuh)
+const char *grad_unsupported(const b200ms_problem &p, const ProblemSetup &s) {
+  if (s.tensorial) return "grad_eps: tensorial (angled or off-diagonal eps) problems are not supported";
+  if (!std::isnan(p.bend_radius)) return "grad_eps: bent waveguides are not supported";
+  if (p.mu || p.incidence) return "grad_eps: mu_cross / split_curl_scaling are not supported";
+  if (s.relative) return "grad_eps: the relative mode solver (basis fields) is not supported";
+  if (s.has_pec) return "grad_eps: problems with PEC-valued cells are not supported";
+  return nullptr;
+}
+
 template <typename T, typename C, typename P, typename PC>
 void solve_group(b200ms_handle *h, const std::vector<int> &ids, const Window &W, const b200ms_problem *prob, b200ms_result *res,
-                 unsigned char *out_region, std::vector<FieldCopy> &copies) {
+                 unsigned char *out_region, const std::vector<cplx *> &grad_dst, std::vector<FieldCopy> &copies) {
   // ids index into the window (global problem index = W.i0 + id)
   const int B = (int)ids.size();
   std::vector<const ProblemSetup *> ps(B);
@@ -737,6 +747,10 @@ void solve_group(b200ms_handle *h, const std::vector<int> &ids, const Window &W,
     if (rb.fields || rb.flux || rb.te_fraction || rb.overlap_prev || prob[W.i0 + ids[b]].post) want_fields = true;  // post-processing needs them in HBM
   }
   S.epilogue(nsorted, perm, ps, nullptr, want_fields);
+  if (std::any_of(grad_dst.begin(), grad_dst.end(), [](cplx *p) { return p != nullptr; })) {
+    NvtxRange r("b200ms:permittivity gradient");
+    S.sensitivity(nsorted, ps, grad_dst);
+  }
   // true residuals on the sorted Ritz vectors (they sit in the FGMRES Z scratch after the permutation)
   std::vector<double> maxres(B, 0.0);
   {
@@ -756,6 +770,8 @@ void solve_group(b200ms_handle *h, const std::vector<int> &ids, const Window &W,
   if (want_fields)
     for (int b = 0; b < B; ++b)
       if (res[W.i0 + ids[b]].fields) copies.push_back({res[W.i0 + ids[b]].fields, out_region + (size_t)b * per, per});
+  for (int b = 0; b < B; ++b)
+    if (grad_dst[b]) copies.push_back({res[W.i0 + ids[b]].grad_eps, grad_dst[b], (size_t)3 * S.N * k * sizeof(cplx)});
   h->stats.device_ms += ms;
   h->stats.launches += S.stats.launches;
   h->stats.inner_iters += (long long)S.stats.inner_iters * B;
@@ -864,17 +880,19 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
           res[i].converged = 0;
         }
         std::map<GroupKey, std::vector<int>> groups;
-        size_t out_bytes = 0;
+        size_t out_bytes = 0, grad_bytes = 0;
         for (int q = 0; q < i1 - i0; ++q) {
           const int i = i0 + q;
           const ProblemSetup &s = W.setups[q];
           if (res[i].status == B200MS_OK) res[i].status = s.status;
           res[i].eps_spec = s.eps_spec;
           res[i].is_complex = s.is_complex;
+          const char *no_grad = (res[i].status == B200MS_OK && res[i].grad_eps) ? grad_unsupported(prob[i], s) : nullptr;
+          if (no_grad) res[i].status = B200MS_ERR_UNSUPPORTED;
           if (res[i].status != B200MS_OK) {
             if (first_err == B200MS_OK) {
               first_err = res[i].status;
-              h->err = s.error.empty() ? "bad result buffers" : s.error;
+              h->err = no_grad ? no_grad : s.error.empty() ? "bad result buffers" : s.error;
             }
             continue;
           }
@@ -883,9 +901,11 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
                        s.masked ? 1 : 0, prob[i].angle_theta, prob[i].angle_phi};
           groups[key].push_back(q);
           out_bytes += align256((size_t)6 * s.nx * s.ny * s.num_modes * (prob[i].precision == 1 ? 8 : 16));
+          if (res[i].grad_eps) grad_bytes += align256((size_t)3 * s.nx * s.ny * s.num_modes * sizeof(cplx));
         }
         DevBuf &ob = h->out[wi & 1];  // last read by the delivery of window wi-2, which has completed (see below)
-        ob.reserve(std::max<size_t>(out_bytes + 4096, 4096));
+        ob.reserve(std::max<size_t>(out_bytes + grad_bytes + 4096, 4096));
+        size_t gcursor = out_bytes;  // permittivity gradients follow the packed fields
         CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
         free_b += h->arena.cap;
         std::vector<FieldCopy> copies;
@@ -900,8 +920,16 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
             const size_t pb = (size_t)6 * sg.nx * sg.ny * sg.num_modes * (prob[i0 + ids[0]].precision == 1 ? 8 : 16);
             unsigned char *region = ob.p + cursor;
             if (cursor + pb * ids.size() > ob.cap) throw std::runtime_error("output buffer accounting error");
+            std::vector<cplx *> grad_dst(ids.size(), nullptr);
+            size_t gc = gcursor;
+            for (size_t b = 0; b < ids.size(); ++b)
+              if (res[i0 + ids[b]].grad_eps) {
+                grad_dst[b] = reinterpret_cast<cplx *>(ob.p + gc);
+                gc += align256((size_t)3 * sg.nx * sg.ny * sg.num_modes * sizeof(cplx));
+              }
+            if (gc > ob.cap) throw std::runtime_error("output buffer accounting error");
             try {
-              dispatch_group(kv.first.kind, h, ids, W, prob, res, region, copies);
+              dispatch_group(kv.first.kind, h, ids, W, prob, res, region, grad_dst, copies);
             } catch (const DeviceOutOfMemory &) {
               // bytes_per_problem is an estimate (other processes, fragmentation): the arena is reserved before anything else
               // of the batch happens, so the same problems are simply solved in smaller device batches
@@ -912,6 +940,7 @@ extern "C" int b200ms_solve_batch(b200ms_handle *h, int nprob, const b200ms_prob
               continue;
             }
             s0 += ids.size();
+            gcursor = gc;
             {
               NvtxRange r("b200ms:post-processing in HBM");
               post_batch(h, ids, W, prob, res, region, pb);  // gauge / flux / normalisation in HBM, before delivery
@@ -993,8 +1022,20 @@ static void bench_group(b200ms_handle *h, const Window &W, int nbatch, int mode,
     for (int q = 0; q < 5; ++q)
       for (int b = 0; b < nbatch; ++b)
         CUDA_CHECK(cudaMemcpyAsync(gsV + (size_t)q * S.vstride + (size_t)b * len, hp.data(), len * sizeof(P), cudaMemcpyHostToDevice, h->stream));
+  // mode 3: the permittivity-gradient kernels, every mode slot holding the random vector, n = 2 for every mode
+  cplx *gdst = nullptr;
+  if (mode == 3) {
+    for (int q = 0; q < S.k; ++q)
+      for (int b = 0; b < nbatch; ++b)
+        CUDA_CHECK(cudaMemcpyAsync(S.gmres_z() + (size_t)q * S.vstride + (size_t)b * len, hx.data(), len * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+    CUDA_CHECK(cudaMalloc(&gdst, (size_t)nbatch * S.k * 3 * S.N * sizeof(cplx)));
+    std::vector<cplx *> dst(nbatch);
+    for (int b = 0; b < nbatch; ++b) dst[b] = gdst + (size_t)b * S.k * 3 * S.N;
+    S.sensitivity_upload(std::vector<cd>((size_t)nbatch * S.k, cd(2.0, 0.0)), ps, dst);
+  }
   auto run = [&]() {
-    if (mode == 2) S.template gs_cgs2<P>(gsV, S.vstride, len, 4, gsW, gsW, nullptr, reinterpret_cast<P *>(S.hessenberg()), (size_t)S.restart * (S.restart + 4));
+    if (mode == 3) S.sensitivity_launch();
+    else if (mode == 2) S.template gs_cgs2<P>(gsV, S.vstride, len, 4, gsW, gsW, nullptr, reinterpret_cast<P *>(S.hessenberg()), (size_t)S.restart * (S.restart + 4));
     else if (mode == 1) S.apply(0, MODE_JACOBI, px, prhs, py);
     else S.apply_true(MODE_APPLY, dx, drhs, dy);
   };
@@ -1021,11 +1062,14 @@ static void bench_group(b200ms_handle *h, const Window &W, int nbatch, int mode,
     total = ms;
   }
   CUDA_CHECK(cudaGetLastError());
+  if (gdst) CUDA_CHECK(cudaFree(gdst));
   if (ms_out) *ms_out = total / nrep;
   // algorithmic bytes (SURVEY 8(d)): apply = read v (2) + write Av (2) + nf coefficient fields per cell;
   // smoother sweep = read x, rhs, omega/diag (6) + write x' (2) + nf coefficient fields per cell
   const double ncell = (double)S.N * nbatch;
-  if (bytes_out && mode == 2)  // dots: 4+1 vectors; update+dots: 4 + r/w w; update+norm: 4 + r/w w; scale: r + w
+  if (bytes_out && mode == 3)  // scan and write pass each read v (2) + exx, eyy, iez per cell and mode; write 3 complex128
+    *bytes_out = ncell * S.k * (2.0 * (2.0 * sizeof(T) + 3.0 * sizeof(C)) + 3.0 * sizeof(cplx));
+  else if (bytes_out && mode == 2)  // dots: 4+1 vectors; update+dots: 4 + r/w w; update+norm: 4 + r/w w; scale: r + w
     *bytes_out = (double)len * nbatch * sizeof(P) * 19.0;
   else if (bytes_out)
     *bytes_out = mode == 1 ? ncell * (8.0 * sizeof(P) + (double)S.nf * sizeof(PC)) : ncell * (4.0 * sizeof(T) + (double)S.nf * sizeof(C));
@@ -1091,6 +1135,61 @@ extern "C" int b200ms_debug_schur(int n, const double *a, double *t, double *q) 
     q[2 * i + 1] = Q.a[i].imag();
   }
   return ok ? B200MS_OK : B200MS_ERR_NOCONV;
+}
+
+extern "C" int b200ms_debug_sensitivity(const b200ms_problem *prob, const double *vec, const double *lambda, double *out) {
+  if (!prob || !vec || !lambda || !out) return B200MS_ERR_ARG;
+  ProblemSetup s;
+  setup_problem(*prob, s);
+  if (s.status != B200MS_OK) return s.status;
+  if (grad_unsupported(*prob, s)) return B200MS_ERR_UNSUPPORTED;
+  const int nx = s.nx, ny = s.ny;
+  const size_t N = (size_t)nx * ny;
+  // the device operands of sensitivity(): 1-D coefficients, exx, eyy, 1 / ezz (the host mirror stores ezz), Yee lengths
+  std::vector<cplx> cx(4 * nx), cy(4 * ny), f(3 * N), len[2];
+  for (int a = 0; a < 2; ++a) {
+    std::vector<cd> c;
+    s.ax[a].coefficients(c);
+    cplx *dst = a == 0 ? cx.data() : cy.data();
+    for (size_t i = 0; i < c.size(); ++i) dst[i] = mk(c[i].real(), c[i].imag());
+    const Axis &A = s.ax[a];
+    len[a].resize(2 * A.n);
+    for (int i = 0; i < A.n; ++i) {
+      len[a][i] = mk(A.lf[i].real(), A.lf[i].imag());
+      len[a][A.n + i] = mk(A.lb[i].real(), A.lb[i].imag());
+    }
+    if (A.pmc && A.n > 1) len[a][A.n] = 0.5 * len[a][A.n];
+  }
+  for (size_t i = 0; i < N; ++i) {
+    f[i] = mk(s.f(0)[i].real(), s.f(0)[i].imag());
+    f[N + i] = mk(s.f(1)[i].real(), s.f(1)[i].imag());
+    const cd iez = 1.0 / s.f(2)[i];
+    f[2 * N + i] = mk(iez.real(), iez.imag());
+  }
+  const cplx *v = reinterpret_cast<const cplx *>(vec);
+  const SensCell<cplx, cplx> c{nx, ny, v, v + N, f.data(), f.data() + N, f.data() + 2 * N, nullptr, cx.data(), cy.data()};
+  cplx S = mk(0.0, 0.0);
+  for (int i = 0; i < nx; ++i)
+    for (int j = 0; j < ny; ++j) {
+      cplx e1, e2, q1, q2, u, ax, ay, az;
+      sens_cell(c, i, j, e1, e2, q1, q2, u);
+      sens_areas(len[0].data(), len[1].data(), nx, ny, i, j, ax, ay, az);
+      S += sens_flux_term(ax, ay, e1, e2, q1, q2);
+    }
+  cd n = std::sqrt(-cd(lambda[0], lambda[1]));  // n_complex of the mode (solver.py:884)
+  if (n.real() < 0) n = -n;
+  const cplx nc = mk(n.real(), n.imag()), inv2s = recip(2.0 * S);
+  cplx *o = reinterpret_cast<cplx *>(out);
+  for (int i = 0; i < nx; ++i)
+    for (int j = 0; j < ny; ++j) {
+      cplx e1, e2, q1, q2, u, ax, ay, az, g[3];
+      sens_cell(c, i, j, e1, e2, q1, q2, u);
+      sens_areas(len[0].data(), len[1].data(), nx, ny, i, j, ax, ay, az);
+      sens_grad(nc, inv2s, ax, ay, az, e1, e2, u, g);
+      const size_t t = (size_t)i * ny + j;
+      for (int q = 0; q < 3; ++q) o[q * N + t] = g[q];
+    }
+  return B200MS_OK;
 }
 
 extern "C" int b200ms_debug_setup(const b200ms_problem *prob, double *sigma, int *flags, double *target, double *knorm,

@@ -20,6 +20,7 @@
 #include "coarse_kernel.cuh"
 #include "march2.cuh"
 #include "march2_tma.cuh"
+#include "sensitivity.cuh"
 
 namespace b200ms {
 
@@ -232,6 +233,10 @@ class BatchSolver {
         sz.add<T>(8);
       }
     }
+    // permittivity gradient (sensitivity()): S partials, per-axis lengths, output pointers
+    sz.add<cplx>((size_t)B * k * kSensChunks);
+    sz.add<cplx>((size_t)B * 2 * (nx + ny));
+    sz.add<cplx *>((size_t)B);
     arena_.reserve(sz.total + (1 << 20));
 
     // ---- allocate + upload ----
@@ -1788,6 +1793,50 @@ class BatchSolver {
     else epilogue_kernel<T, C, false><<<grd, blk, 0, st_>>>(a);
     CUDA_CHECK(cudaGetLastError());
   }
+  // dn/deps of every mode of the problems with dst[b] != nullptr (device buffers, [M][3][nx][ny] complex128), from the Ritz
+  // vectors epilogue() left in mode order; ncomplex_sorted as passed to epilogue() (csrc/sensitivity.cuh)
+  void sensitivity(const std::vector<cd> &ncomplex_sorted, const std::vector<const ProblemSetup *> &ps, const std::vector<cplx *> &dst) {
+    sensitivity_upload(ncomplex_sorted, ps, dst);
+    sensitivity_launch();
+    CUDA_CHECK(cudaStreamSynchronize(st_));
+  }
+  void sensitivity_upload(const std::vector<cd> &ncomplex_sorted, const std::vector<const ProblemSetup *> &ps, const std::vector<cplx *> &dst) {
+    if (!sens_part_) {
+      sens_part_ = arena_.get<cplx>((size_t)B * k * kSensChunks);
+      sens_len_ = arena_.get<cplx>((size_t)B * 2 * (nx + ny));
+      sens_out_ = arena_.get<cplx *>((size_t)B);
+    }
+    std::vector<cplx> nh((size_t)B * k), lens((size_t)B * 2 * (nx + ny));
+    for (size_t i = 0; i < nh.size(); ++i) nh[i] = mk(ncomplex_sorted[i].real(), ncomplex_sorted[i].imag());
+    for (int b = 0; b < B; ++b)
+      for (int a = 0; a < 2; ++a) {
+        const Axis &A = ps[b]->ax[a];
+        cplx *l = lens.data() + (a == 0 ? (size_t)b * 2 * nx : (size_t)B * 2 * nx + (size_t)b * 2 * ny);
+        for (int i = 0; i < A.n; ++i) {
+          l[i] = mk(A.lf[i].real(), A.lf[i].imag());
+          l[A.n + i] = mk(A.lb[i].real(), A.lb[i].imag());
+        }
+        if (A.pmc && A.n > 1) l[A.n] = 0.5 * l[A.n];  // the PMC row of Db is 2 / lb[0]: half a dual cell
+      }
+    CUDA_CHECK(cudaMemcpyAsync(ncomplex_, nh.data(), nh.size() * sizeof(cplx), cudaMemcpyHostToDevice, st_));
+    CUDA_CHECK(cudaMemcpyAsync(sens_len_, lens.data(), lens.size() * sizeof(cplx), cudaMemcpyHostToDevice, st_));
+    CUDA_CHECK(cudaMemcpyAsync(sens_out_, dst.data(), (size_t)B * sizeof(cplx *), cudaMemcpyHostToDevice, st_));
+    CUDA_CHECK(cudaStreamSynchronize(st_));  // the host vectors above must outlive the copies
+  }
+  // the two gradient kernels on the vectors in gmres_z() (epilogue() leaves the Ritz vectors there in mode order)
+  void sensitivity_launch() {
+    SensArgs<T, C> a;
+    a.nx = nx; a.ny = ny; a.num_modes = k; a.vec = Zg_; a.vstride = vstride;
+    a.fields = lv[0].fields_true; a.field_bstride = lv[0].fbstride; a.has_mu = has_mu ? 1 : 0;
+    a.cx = lv[0].cx_true; a.cy = lv[0].cy_true; a.len_x = sens_len_; a.len_y = sens_len_ + (size_t)B * 2 * nx;
+    a.ncomplex = ncomplex_; a.out = sens_out_;
+    sens_scan_kernel<T, C><<<dim3(kSensChunks, B * k), 256, 0, st_>>>(a, sens_part_);
+    CUDA_CHECK(cudaGetLastError());
+    const unsigned nblk = (unsigned)std::min<size_t>((N + 255) / 256, 1024);
+    sens_write_kernel<T, C><<<dim3(nblk, B * k), 256, 0, st_>>>(a, sens_part_);
+    CUDA_CHECK(cudaGetLastError());
+    stats.launches += 2;
+  }
   T *scratch_vec(int i) { return i == 0 ? xsol_ : rhs_; }
   T *basis0() { return Vout_; }
   T *gmres_z() { return Zg_; }
@@ -1907,6 +1956,8 @@ class BatchSolver {
   std::vector<T> hhost_;
   std::vector<cd> sig_host_;
   // round-2 inner solver state
+  cplx *sens_part_ = nullptr, *sens_len_ = nullptr;
+  cplx **sens_out_ = nullptr;
   P *cx_true_p_ = nullptr, *cy_true_p_ = nullptr;  // reference-operator difference coefficients in the multigrid precision
   T *Hd_ = nullptr, *ydev_ = nullptr, *gpart_ = nullptr;
   cplx *lsq_work_ = nullptr;

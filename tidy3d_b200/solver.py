@@ -76,9 +76,29 @@ def _undo_split_curl(fields, split):
     return fields
 
 
+def _check_grad_scope(p: dict):
+    """Raise NotImplementedError when the permittivity gradient of problem ``p`` is outside the diagonal path (DESIGN.md
+    section 10).  What needs the rasterised medium of a ``section`` (off-diagonal or PEC-valued sites) is checked by the library."""
+    ms = p["mode_spec"]
+    if getattr(ms, "bend_radius", None) is not None:
+        raise NotImplementedError("grad_eps: bent waveguides are not supported")
+    if float(getattr(ms, "angle_theta", 0.0)) != 0.0:
+        raise NotImplementedError("grad_eps: angled problems are not supported")
+    for key in ("mu_cross", "split_curl_scaling", "solver_basis_fields"):
+        if p.get(key) is not None:
+            raise NotImplementedError(f"grad_eps: problems with {key} are not supported")
+    if p.get("eps_cross") is not None:
+        ec = p["eps_cross"]
+        ec = ec if isinstance(ec, np.ndarray) else np.array([np.asarray(c) for c in ec])
+        if np.any(np.abs(ec) >= 0.9 * abs(PEC_VAL)):
+            raise NotImplementedError("grad_eps: problems with PEC-valued cells are not supported")
+        if np.any(np.abs(ec[[1, 2, 3, 5, 6, 7]]) > 1e-6):  # the tensorial test of solver.py:336-339
+            raise NotImplementedError("grad_eps: tensorial (off-diagonal eps) problems are not supported")
+
+
 def compute_modes_batch(
     problems: Sequence[dict], device: int = -1, want_fields: bool = True, return_info: bool = False, handle=None,
-    fields_ptrs=None, post: Optional[Sequence[str]] = None,
+    fields_ptrs=None, post: Optional[Sequence[str]] = None, grad_eps=False, grad_eps_ptrs=None,
 ):
     """Solve many independent mode problems in one device call.
 
@@ -98,8 +118,26 @@ def compute_modes_batch(
     finite-grid correction factors of ``ModeSolver._grid_correction`` (mode_solver.py:847-904), like the reference's; and
     ``plane_bounds=(xmin, xmax, ymin, ymax)`` (``plugin.plane_bounds_of``): the extent of a finite mode plane, to which the
     integration weights are truncated like the reference's ``_diff_area`` (monitor_data.py:437-455).
+
+    ``grad_eps``: True (every problem) or one bool per problem.  The info dict of such a problem then carries ``grad_eps``, an
+    ndarray ``(M, 3, Nx, Ny)`` complex128 = d n_complex[m] / d eps_cross[c, c][ix, iy] for c in xx, yy, zz, from the left
+    eigenvector of the diagonal operator (no extra solve; works with ``want_fields=False``).  ``grad_eps_ptrs``: one raw
+    address per problem (host or device memory, 0 / None = no gradient) the library writes that array to instead.  Only the
+    diagonal path is differentiable: bends, angles, off-diagonal eps, ``mu_cross``, ``split_curl_scaling``,
+    ``solver_basis_fields`` and PEC-valued cells raise NotImplementedError.
     """
     post = tuple(post or ())
+    if grad_eps_ptrs is not None:
+        want_grad = [bool(a) for a in grad_eps_ptrs]
+    elif isinstance(grad_eps, (bool, np.bool_)):
+        want_grad = [bool(grad_eps)] * len(problems)
+    else:
+        want_grad = [bool(g) for g in grad_eps]
+    if len(want_grad) != len(problems):
+        raise ValueError("grad_eps / grad_eps_ptrs need one entry per problem")
+    for p, g in zip(problems, want_grad):
+        if g:
+            _check_grad_scope(p)
     unknown = set(post) - {"gauge", "normalize", "flux", "overlaps"}
     if unknown:
         raise ValueError(f"unknown post-processing step(s): {sorted(unknown)}")
@@ -139,9 +177,11 @@ def compute_modes_batch(
         packed.append(pk)
     h = handle or get_handle(device)  # after input validation: argument errors do not need a GPU
     with h.lock:
+        grad_kw = dict(grad_eps=want_grad, grad_eps_ptrs=grad_eps_ptrs) if any(want_grad) else {}
         rc, fields, ncs, results = h.solve_batch(packed, want_fields, fields_ptrs, want_flux=("flux" in post or "normalize" in post),
-                                                 want_overlaps="overlaps" in post)
+                                                 want_overlaps="overlaps" in post, **grad_kw)
         flux_out, te_out, ov_out = h.last_flux, h.last_te, h.last_overlaps
+        grad_out = h.last_grad if grad_kw else [None] * len(packed)
         err = h.last_error() if rc != _cabi.OK else ""
     if rc != _cabi.OK:
         bad = [i for i in range(len(packed)) if results[i].status != _cabi.OK]
@@ -163,6 +203,8 @@ def compute_modes_batch(
             infos[-1]["te_fraction"] = te_out[i]
         if ov_out:
             infos[-1]["overlap_prev"] = ov_out[i]
+        if grad_out[i] is not None:
+            infos[-1]["grad_eps"] = grad_out[i]
     return (out, infos) if return_info else out
 
 
